@@ -21,6 +21,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (no __pycache__ beside the sources)
 for p in (ROOT, os.path.join(ROOT, 'sd-webui-text2video_b200')):
     if p not in sys.path:
         sys.path.insert(0, p)
@@ -51,7 +52,31 @@ def parse():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-gpu-baseline', action='store_true', help='skip the torch-eager GPU comparator leg of the N=1 run')
     ap.add_argument('--cpu-frames', type=int, default=0, help='frames of the CPU sample (0 = the metric\'s F)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed clips, write what the last one returned (the '
+                                                          'decoded uint8 frames) to DIR/<name>.npy as float32')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be >= 1')
+    return args
+
+
+DUMP_LIMIT_BYTES = 60 << 20     # all dumped arrays together stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor as out_dir/<name>.npy in float32.  When the arrays together exceed DUMP_LIMIT_BYTES, each is
+    replaced by the same share of its flattened elements at indices drawn from a fixed seed (sorted), so two runs with
+    the same arguments dump the same positions."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.numel() for a in arrays.values())
+    budget = DUMP_LIMIT_BYTES // 4
+    for name, a in arrays.items():
+        a = a.detach().float().cpu().numpy()
+        if total > budget:
+            idx = np.sort(np.random.default_rng(0).integers(0, a.size, a.size * budget // total))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def peaks():
@@ -329,6 +354,7 @@ def run_b200(args):
             dist.all_gather(out, frames_u8)
 
     def timed(fn, k, base_seed, with_gather):
+        """(ms for k clips, what the last clip returned)"""
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
@@ -344,7 +370,7 @@ def run_b200(args):
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
             dist.barrier()
-        return float(ms.item())
+        return float(ms.item()), r
 
     from t2v_b200 import distributed as D
     unit, n_units = D.units()       # clip-rendering units: ranks (sample-DP) or rank pairs (T2V_CFG_SPLIT=1, distributed.py)
@@ -356,12 +382,14 @@ def run_b200(args):
     torch.cuda.synchronize()
     clk = ClockSampler(local)
     clk.start()
-    ms = timed(clip_device, args.steps, 123, True)
+    ms, last_frames = timed(clip_device, args.steps, 123, True)
     clk.stop_flag = True
     clk.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'frames': last_frames})
     fps = n_units * args.steps * F / (ms / 1000.0)
     clip_e2e(7)                                   # warm the e2e path (pinned staging, plan for B=2 already built)
-    ms_e2e = timed(clip_e2e, args.steps, 123, False)
+    ms_e2e, _ = timed(clip_e2e, args.steps, 123, False)
     fps_e2e = n_units * args.steps * F / (ms_e2e / 1000.0)
 
     prof = None

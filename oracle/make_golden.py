@@ -25,6 +25,9 @@ from oracle import samplers_oracle as SO                      # noqa: E402
 from oracle import vc_oracle as VC                            # noqa: E402
 
 GOLD = os.path.join(ROOT, 'tests', 'golden')
+# fixture files stay under 1 MB: the full-size single-step fixture keeps every X1_STRIDE-th element of its three
+# after-one-update latents (7 is odd, so the sample walks through every row, column, frame and channel)
+X1_STRIDE = 7
 
 
 def build_ref_unet(m, cfg: UO.UNetConfig):
@@ -258,6 +261,10 @@ def gold_unet_step(m, name, cfg, F, h, w, wseed, unipc=True):
         d = (om.calls[-1] - out[key]).abs().max().item()
         print(f'[{name}] {key}: oracle-sampler-vs-reference max|d| = {d:.3e}', flush=True)
         assert d < 5e-4, (key, d)
+    for key in ('ddim_gaussian_x1', 'ddim_x1', 'unipc_x1'):
+        if key in out:
+            out[key] = out[key].reshape(-1)[::X1_STRIDE].clone()
+    out['x1_stride'] = X1_STRIDE
     torch.save(out, os.path.join(GOLD, name + '.pt'))
     return out
 
@@ -517,6 +524,68 @@ def gold_vid2vid_encode():
     torch.save(out, os.path.join(GOLD, 'vid2vid_encode.pt'))
 
 
+def gold_module_tree(m):
+    """State-dict shapes of the reference's UNetSD (dim 64) and AutoencoderKL, and the class of each Linear / Conv
+    module of the UNet: the layout the nn.Module mirrors must expose (tests/test_modules_cpu.py)."""
+    ddconfig = {'double_z': True, 'z_channels': 4, 'resolution': 256, 'in_channels': 3, 'out_ch': 3, 'ch': 128,
+                'ch_mult': [1, 2, 4, 4], 'num_res_blocks': 2, 'attn_resolutions': [], 'dropout': 0.0}
+    torch.manual_seed(0)
+    net = build_ref_unet(m, UO.UNetConfig(dim=64))
+    kinds = ('Linear', 'Conv1d', 'Conv2d', 'Conv3d')
+    ae = m.AutoencoderKL(ddconfig, 4, None)
+    out = {'unet_dim64': {'state_dict': {k: tuple(v.shape) for k, v in net.state_dict().items()},
+                          'modules': {n: type(x).__name__ for n, x in net.named_modules() if type(x).__name__ in kinds}},
+           'vae': {'state_dict': {k: tuple(v.shape) for k, v in ae.state_dict().items()}}}
+    torch.save(out, os.path.join(GOLD, 'module_tree.pt'))
+    print(f'[module_tree] unet {len(out["unet_dim64"]["state_dict"])} tensors, vae {len(out["vae"]["state_dict"])} tensors')
+
+
+def gold_unet_tiny_b2(m):
+    """The reference UNetSD (dim 64) at B = 2 with two different timesteps, seeded weights and inputs."""
+    cfg = UO.UNetConfig(dim=64)
+    torch.manual_seed(0)
+    net = build_ref_unet(m, cfg)
+    W = UO.make_weights(UO.param_specs(cfg), seed=5)
+    net.load_state_dict(W, strict=True)
+    g = torch.Generator().manual_seed(9)
+    x = torch.randn(2, 4, 3, 8, 8, generator=g)
+    y = torch.randn(2, 77, 1024, generator=g)
+    t = torch.tensor([500, 20])
+    with torch.no_grad():
+        ref = net(x, t, y)
+    err = (UO.unet_forward(W, cfg, x, t, y) - ref).abs().max().item()
+    print(f'[unet_tiny_b2] oracle-vs-reference max|d| = {err:.3e}')
+    torch.save({'wseed': 5, 'xy_seed': 9, 'x_shape': tuple(x.shape), 'y_shape': tuple(y.shape), 't': t, 'out': ref},
+               os.path.join(GOLD, 'unet_tiny_b2.pt'))
+
+
+KEY_FRAME_CASES = [
+    (8, 4, '0:(t/max_i_f), "max_i_f":(1)'), (24, 8, '0:(t/max_i_f), "max_i_f":(1)'), (6, 4, '0:(0.25), 3:(1.0)'),
+    (10, 3, '0:(0), 4:(0.5), "max_f":(1)'), (12, 6, '0:(sin(t/max_f)), 9:(0.2)'),
+    (8, 4, '0:(t/max_i_f), "max_i_f":(1*1)'), (16, 5, '0:(0.1+t/max_f), 11:(t*t/(max_f*max_f))')]
+
+
+def gold_key_frames():
+    """Per-frame inpainting weights of the reference's T2VAnimKeys (t2v_helpers/key_frames.py) for KEY_FRAME_CASES.
+    A spec the reference cannot evaluate with the installed pandas is stored with weights None: numeric keys make it
+    store a string into a float64 Series (key_frames.py:38), which pandas >= 3 rejects with a TypeError."""
+    import json
+    import pandas
+    from types import SimpleNamespace as NS
+    kf = ref_shim.load_key_frames()
+    cases = []
+    for frames, i_frames, spec in KEY_FRAME_CASES:
+        try:
+            w = [float(v) for v in kf.T2VAnimKeys(NS(max_frames=frames, inpainting_weights=spec), 7, i_frames)
+                 .inpainting_weights_series]
+        except TypeError:
+            w = None
+        cases.append({'frames': frames, 'i_frames': i_frames, 'spec': spec, 'weights': w})
+    with open(os.path.join(GOLD, 'key_frames.json'), 'w') as f:
+        json.dump({'pandas': pandas.__version__, 'cases': cases}, f, indent=1)
+    print(f'[key_frames] {sum(c["weights"] is not None for c in cases)} of {len(cases)} specs evaluated by the reference')
+
+
 def main(only=None):
     os.makedirs(GOLD, exist_ok=True)
     m = ref_shim.load_modelscope()
@@ -529,6 +598,12 @@ def main(only=None):
         gold_vae_encode(m)
     if want('vid2vid_encode'):
         gold_vid2vid_encode()
+    if want('module_tree'):
+        gold_module_tree(m)
+    if want('unet_tiny_b2'):
+        gold_unet_tiny_b2(m)
+    if want('key_frames'):
+        gold_key_frames()
     tiny = UO.UNetConfig(dim=64)
     keep = ['input_blocks.0.0', 'input_blocks.0.1', 'input_blocks.1.0', 'input_blocks.1.1', 'input_blocks.1.2',
             'input_blocks.3', 'input_blocks.4.0', 'input_blocks.11.0', 'middle_block.1', 'middle_block.3',

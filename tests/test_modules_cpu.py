@@ -1,12 +1,12 @@
 """CPU: the nn.Module mirrors expose the reference's state_dict / module tree (load_state_dict(strict=True), LoRA
 name matching) and schedule buffers -- checked against the oracle's parameter table (itself pinned against the
-reference) and, when mounted, against the reference classes directly."""
+reference) and against the reference classes' own layout, stored in tests/golden."""
 import numpy as np
 import pytest
 import torch
 import torch.nn as nn
 
-from oracle import unet_oracle as UO, vae_oracle as VO, ref_shim
+from oracle import unet_oracle as UO, vae_oracle as VO
 from oracle import samplers_oracle as SO
 from t2v_b200.modules import UNetSD, AutoencoderKL
 from t2v_b200.pipeline import VAE_DDCONFIG, linear_sd_betas
@@ -69,20 +69,18 @@ def test_cpu_forward_is_refused():
         net(torch.zeros(1, 4, 2, 8, 8), torch.tensor([1]), torch.zeros(1, 77, 1024))
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason='reference tree not mounted')
-def test_mirror_against_reference_classes():
-    m = ref_shim.load_modelscope()
-    ref = m.UNetSD(in_dim=4, dim=64, y_dim=768, context_dim=1024, out_dim=4, dim_mult=[1, 2, 4, 4], num_heads=8,
-                   head_dim=64, num_res_blocks=2, attn_scales=[1, 0.5, 0.25], dropout=0.1, temporal_attention=True)
+def test_mirror_against_reference_classes(gold_dir):
+    """State-dict shapes and Linear / Conv classes of the mirrors vs the reference's UNetSD (dim 64) and AutoencoderKL
+    (tests/golden/module_tree.pt, written by oracle/make_golden.py from the reference classes)."""
+    import os
+    ref = torch.load(os.path.join(gold_dir, 'module_tree.pt'))
     mine = UNetSD(dim=64)
-    assert {k: tuple(v.shape) for k, v in ref.state_dict().items()} == {k: tuple(v.shape) for k, v in mine.state_dict().items()}
+    assert ref['unet_dim64']['state_dict'] == {k: tuple(v.shape) for k, v in mine.state_dict().items()}
     kinds = ('Linear', 'Conv1d', 'Conv2d', 'Conv3d')
-    rt = {n: type(x).__name__ for n, x in ref.named_modules() if type(x).__name__ in kinds}
     mt = {n: type(x).__name__ for n, x in mine.named_modules() if type(x).__name__ in kinds}
-    assert rt == mt
-    rv = m.AutoencoderKL(dict(VAE_DDCONFIG), 4, None)
+    assert ref['unet_dim64']['modules'] == mt
     mv = AutoencoderKL(VAE_DDCONFIG, 4)
-    assert {k: tuple(v.shape) for k, v in rv.state_dict().items()} == {k: tuple(v.shape) for k, v in mv.state_dict().items()}
+    assert ref['vae']['state_dict'] == {k: tuple(v.shape) for k, v in mv.state_dict().items()}
 
 
 # ---------------------------------------------------------------------------------------- VideoCrafter mirrors
@@ -154,7 +152,7 @@ def test_vid2vid_entry_noise_matches_reference_fixture(gold_dir, strength, steps
     (8, 4, '0:(t/max_i_f), "max_i_f":(1)'), (24, 8, '0:(t/max_i_f), "max_i_f":(1)'), (6, 4, '0:(0.25), 3:(1.0)'),
     (10, 3, '0:(0), 4:(0.5), "max_f":(1)'), (12, 6, '0:(sin(t/max_f)), 9:(0.2)'),
     (8, 4, '0:(t/max_i_f), "max_i_f":(1*1)'), (16, 5, '0:(0.1+t/max_f), 11:(t*t/(max_f*max_f))')])
-def test_inpainting_weight_schedule_matches_reference(frames, i_frames, spec):
+def test_inpainting_weight_schedule_matches_reference(gold_dir, frames, i_frames, spec):
     """T2VAnimKeys (t2v_helpers/key_frames.py:9-95) restated without numexpr / pandas: same per-frame weights, including the
     reference's 'expression sticks until the next numeric key' behaviour."""
     from types import SimpleNamespace as NS
@@ -166,18 +164,19 @@ def test_inpainting_weight_schedule_matches_reference(frames, i_frames, spec):
     }.get((frames, i_frames, spec))
     if expected is not None:
         assert np.allclose(got, expected)
-    from oracle import ref_shim
-    if ref_shim.reference_available():                                   # live against the unmodified reference class
-        kf = ref_shim.load_key_frames()
-        try:
-            ref = kf.T2VAnimKeys(NS(max_frames=frames, inpainting_weights=spec), 7, i_frames).inpainting_weights_series
-        except TypeError:
-            # numeric keys: the reference stores the STRING into a float64 Series (key_frames.py:38), which pandas >= 3 (3.0.2
-            # here) rejects -- the unmodified reference cannot run those specs in this container; the expression-valued
-            # specs below it are compared live
-            assert any(ch.isdigit() for ch in spec)
-            return
-        assert np.allclose(got, np.asarray(ref, dtype=np.float64), rtol=0, atol=1e-12)
+    # the unmodified reference class's weights for the same spec (tests/golden/key_frames.json, oracle/make_golden.py)
+    import json
+    import os
+    with open(os.path.join(gold_dir, 'key_frames.json')) as f:
+        ref = [c['weights'] for c in json.load(f)['cases'] if (c['frames'], c['i_frames'], c['spec']) == (frames, i_frames, spec)]
+    assert len(ref) == 1
+    if ref[0] is None:
+        # numeric keys: the reference stores the STRING into a float64 Series (key_frames.py:38), which pandas >= 3
+        # rejects -- the unmodified reference could not run those specs when the fixture was written; the
+        # expression-valued specs are compared
+        assert any(ch.isdigit() for ch in spec)
+        return
+    assert np.allclose(got, np.asarray(ref[0], dtype=np.float64), rtol=0, atol=1e-12)
 
 
 def test_stable_lora_processor_walk_and_flags_on_cpu():

@@ -1,13 +1,11 @@
 """CPU: the oracle restatement reproduces the committed reference outputs (tests/golden/*.pt, produced by
-oracle/make_golden.py from the UNMODIFIED reference).  When /root/reference is mounted, the restatement is also
-re-checked live against the reference modules."""
+oracle/make_golden.py from the UNMODIFIED reference)."""
 import os
 
 import pytest
 import torch
 
 from oracle import unet_oracle as UO, vae_oracle as VO, samplers_oracle as SO
-from oracle import ref_shim
 from oracle.make_golden import analytic_model, _SchedModel, synth_inputs
 
 
@@ -81,21 +79,15 @@ def test_ddim_timestep_grids():
     assert dts[0] == 1 and dts[-1] == 981
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason='reference tree not mounted')
-def test_oracle_unet_live_against_reference():
-    m = ref_shim.load_modelscope()
+def test_oracle_unet_live_against_reference(gold_dir):
+    """B = 2 with two different timesteps: oracle vs the reference UNetSD's output (tests/golden/unet_tiny_b2.pt)."""
+    g = torch.load(os.path.join(gold_dir, 'unet_tiny_b2.pt'))
     cfg = UO.UNetConfig(dim=64)
-    net = m.UNetSD(in_dim=4, dim=64, y_dim=768, context_dim=1024, out_dim=4, dim_mult=[1, 2, 4, 4], num_heads=8,
-                   head_dim=64, num_res_blocks=2, attn_scales=[1, 0.5, 0.25], dropout=0.1, temporal_attention=True).eval()
-    W = UO.make_weights(UO.param_specs(cfg), seed=5)
-    net.load_state_dict(W, strict=True)
-    g = torch.Generator().manual_seed(9)
-    x = torch.randn(2, 4, 3, 8, 8, generator=g)
-    y = torch.randn(2, 77, 1024, generator=g)
-    t = torch.tensor([500, 20])
-    with torch.no_grad():
-        ref = net(x, t, y)
-    assert torch.allclose(UO.unet_forward(W, cfg, x, t, y), ref, rtol=0, atol=3e-5)
+    W = UO.make_weights(UO.param_specs(cfg), seed=g['wseed'])
+    gen = torch.Generator().manual_seed(g['xy_seed'])
+    x = torch.randn(g['x_shape'], generator=gen)
+    y = torch.randn(g['y_shape'], generator=gen)
+    assert torch.allclose(UO.unet_forward(W, cfg, x, g['t'], y), g['out'], rtol=0, atol=3e-5)
 
 
 # ---------------------------------------------------------------------------------------- VideoCrafter (SURVEY.md 8 a19-a20)
@@ -176,9 +168,10 @@ def test_full_size_fixtures_are_consistent(gold_dir):
         SO.ddim_gaussian_sample(model, SO.linear_sd_betas(), x, 50, c, uc, 17.0, trace=tr)
     except StopIteration:
         pass
-    assert torch.allclose(tr[0], g['ddim_gaussian_x1'], rtol=0, atol=1e-6)
+    s = g['x1_stride']                        # the latents after one update are stored as every s-th element
+    assert torch.allclose(tr[0].reshape(-1)[::s], g['ddim_gaussian_x1'], rtol=0, atol=1e-6)
     for k in ('ddim_x1', 'unipc_x1'):
-        assert g[k].shape == x.shape and torch.isfinite(g[k]).all()
+        assert g[k].shape == x.reshape(-1)[::s].shape and torch.isfinite(g[k]).all()
     g3 = torch.load(os.path.join(gold_dir, 'unet_cfg3_slice.pt'))
     assert g3['eps'].shape == (1, 4, 2, 72, 128)
     g5 = torch.load(os.path.join(gold_dir, 'vc_unet_cfg5.pt'))
